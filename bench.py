@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the MeMOTR per-frame hot path on B200 (contract: see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--mode bf16|fp32] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--mode bf16|fp32] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 The hot path of one frame: level flattening + position maps -> 6-layer deformable encoder -> 6-layer decoder (300 detect +
@@ -238,6 +238,24 @@ def gpu_reference_fps(dev, steps, warmup):
     return steps / (s.elapsed_time(e) * 1e-3)
 
 
+def dump_outputs(eng, out_dir):
+    """The arrays a caller receives for the frame the engine ran last: the reference's output dict (FrameEngine.results),
+    the live rows of the track table and the frame's result rows (tracker on the device), or the track state the caller
+    keeps (--no-tracker).  fp32, integer fields as float64 (exact); about 26 MB at the DanceTrack size."""
+    import numpy as np
+    arrays = dict(eng.results())
+    if eng.trk is not None:
+        arrays.update({"track_" + k: v for k, v in eng.table.active().items()})
+        ids, boxes, scores, keep = eng.trk.split_results(eng.trk.res_flat)
+        arrays.update(result_ids=ids, result_boxes=boxes, result_scores=scores, result_keep=keep)
+    else:
+        arrays.update({"track_" + k: v for k, v in eng.st.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        v = v.detach().cpu()
+        np.save(os.path.join(out_dir, k + ".npy"), (v.float() if v.is_floating_point() else v.double()).numpy())
+
+
 def _timeit_us(fn, iters, warmup, flush):
     for _ in range(warmup):
         fn()
@@ -309,11 +327,17 @@ def main():
                     help="upload the position maps with every frame (A/B; default: rebuilt on the device from the masks)")
     ap.add_argument("--no-tracker", action="store_true",
                     help="leave the RuntimeTracker glue out of the step (A/B; default: on the device, inside the graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed frame returned (frame outputs, track table, result rows) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
-    W, K, CLIP = max(args.warmup, 3), max(args.steps, 1), args.clip_frames
+    W, K, CLIP = max(args.warmup, 3), args.steps, args.clip_frames
 
     if args.impl == "reference":
         # the reference's own CPU implementation of the path, host threads, rank 0 only; one step = one frame of the clip
@@ -499,6 +523,8 @@ def main():
     t1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     ms = torch.tensor([t0.elapsed_time(t1)], device=dev)
     ms_all = None
     if world > 1:
